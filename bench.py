@@ -4,6 +4,7 @@ other BASELINE.json configurations as `--workload`s.
 
   python bench.py --gpus 1 --steps 8 --warmup 3                       # config 4 (the headline)
   python bench.py --workload vit_b16_cls | mixer_b16 | vit_s16 | siglip_l14_336
+  python bench.py --dump-outputs DIR ...  # also write the last timed step's outputs as DIR/<name>.npy
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
       --master-port P bench.py --gpus N --steps K --warmup W
   python bench.py --impl reference ...   # the reference's algorithm on the host cores (oracle port)
@@ -283,7 +284,7 @@ def run_reference(args):
   if wl["res"] > 224:
     samples = 2
   warmup = max(1, args.warmup)
-  steps = max(1, args.steps)
+  steps = args.steps
   port = CpuPort(wl, samples, threads)
   t_first = port.step()                              # warm-up step 1 (allocations, MKL plans)
   est = t_first * (warmup - 1 + steps)
@@ -291,8 +292,6 @@ def run_reference(args):
     samples //= 2
     est /= 2
     port = CpuPort(wl, samples, threads)
-  if est > budget_s:                                 # pathological host: keep the run bounded anyway
-    steps = max(1, int(budget_s / (est / (warmup - 1 + steps))) - (warmup - 1))
   for _ in range(warmup - 1):
     port.step()
   t = sum(port.step() for _ in range(steps))
@@ -386,6 +385,34 @@ def run_torch_gpu(args):
 # ----------------------------------------------------------------------------------------------
 # our arm
 # ----------------------------------------------------------------------------------------------
+DUMP_SAMPLE = 1 << 21     # train-state elements per array written by --dump-outputs (8 MB in float32)
+
+
+def dump_outputs(out_dir, state, measurements):
+  """Writes what update_fn handed back to its caller in its last step, one .npy file per array: every
+  measurement and the optimizer's step count in full, and the parameters, their gradients and Adam's two
+  moments at the same DUMP_SAMPLE positions.  The positions are drawn with a fixed seed over the parameters
+  concatenated in name order, so they do not depend on the flat buffer's layout; ~32 MB in all."""
+  import numpy as np
+  import torch
+  P, opt = state["params"], state["opt"]
+  names = sorted(P.offsets)
+  sizes = np.array([int(np.prod(P.offsets[k][1])) for k in names])
+  starts = np.cumsum(sizes) - sizes
+  pos = np.sort(np.random.default_rng(0).choice(int(sizes.sum()), size=min(DUMP_SAMPLE, int(sizes.sum())),
+                                                replace=False))
+  which = np.searchsorted(starts, pos, side="right") - 1
+  idx = torch.from_numpy(np.array([P.offsets[k][0] for k in names])[which] + (pos - starts[which]))
+  idx = idx.to(P.flat.device)
+  # the moments are packed over the trained ranges of the flat buffer: all of it, as OPT_CONFIG freezes nothing
+  assert opt["mu"].numel() == opt["nu"].numel() == P.total
+  arrays = dict(measurements, params=P.flat[idx], grads=P.grad[idx], adam_mu=opt["mu"][idx], adam_nu=opt["nu"][idx])
+  os.makedirs(out_dir, exist_ok=True)
+  for k, v in arrays.items():
+    np.save(os.path.join(out_dir, k + ".npy"), v.float().cpu().numpy())
+  np.save(os.path.join(out_dir, "opt_count.npy"), np.float64(opt["count"]))
+
+
 def measure_ours(args, wl, world, rank, local_rank):
   """Builds the model, runs the device-resident and the end-to-end timed regions; returns a dict of
   raw measurements.  Everything that owns device memory is local to this function, so it is released
@@ -456,6 +483,8 @@ def measure_ours(args, wl, world, rank, local_rank):
   ev1.record()
   barrier()
   launches = L.LAUNCHES[0] - launches0
+  if args.dump_outputs and rank == 0:
+    dump_outputs(args.dump_outputs, state, m)
   # (2) the same K steps again with a CUDA-event pair around every GEMM launch (the roofline's
   # `achieved`); kept apart from (1) so that the event records are not inside the headline number
   ops.gemm = timed_gemm
@@ -646,7 +675,14 @@ def main():
   ap.add_argument("--no-gpu-baseline", action="store_true")
   ap.add_argument("--profile-calls", action="store_true",
                   help="time every C-ABI call of one extra step with CUDA events; breakdown on stderr")
+  ap.add_argument("--dump-outputs", metavar="DIR",
+                  help="after the timed steps, write what the last of them returned (measurements, step count, "
+                       "a fixed sample of parameters, gradients and Adam moments) as DIR/<name>.npy")
   args = ap.parse_args()
+  if args.steps < 1:
+    ap.error("--steps must be at least 1")
+  if args.dump_outputs and args.impl != "ours":
+    ap.error("--dump-outputs applies to --impl ours")
   if args.impl == "reference":
     run_reference(args)
   elif args.impl == "torch_gpu":

@@ -23,8 +23,8 @@ vectors for this path (SURVEY.md 8c).  What pins this file instead:
     logits, loss and parameter gradients (1e-6 relative) for the two-tower model with MAP head and
     last-token text pooling, and the same logits (1e-9), softmax / sigmoid cross-entropies and gradients
     (1e-8) for the cls-token classifier; the committed golden vectors the GPU tests use
-    (tests/golden/siglip_tiny.npz) are reproduced by SiglipModel from the file's own parameters and
-    inputs.  This is not the reference itself, so the "unpinned" label
+    (tests/golden/siglip_tiny.npz) are reproduced by SiglipModel from the parameters and inputs whose
+    digests the file stores.  This is not the reference itself, so the "unpinned" label
     stays; it does pin every flax default listed above plus the [d, h, dh] head split, the MAP head,
     the class-token / position-embedding order and both losses against an implementation that
     reproduces the reference's checkpoints.  Not covered by it: MLP-Mixer, sincos2d, gap / "0" pooling,

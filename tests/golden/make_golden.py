@@ -1,8 +1,10 @@
 """Generates tests/golden/siglip_tiny.npz with the CPU oracle (float64).
 
-No JAX/flax is installable here or on the GPU box, so these vectors come from oracle/bv_oracle.py
+JAX/flax are not dependencies of this project, so these vectors come from oracle/bv_oracle.py
 (itself checked against torch's independent operators in tests/test_oracle.py); they pin the
 oracle against drift and give the GPU tests a fixed target that does not depend on re-running it.
+The parameters (init seed 0) and the image (synthetic recipe, seed 0) are not stored, only their
+digests: tests/common.py:load_golden_tiny regenerates them and checks the digests.
   python tests/golden/make_golden.py
 """
 import os
@@ -15,19 +17,13 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(HERE)))
 sys.path.insert(0, os.path.dirname(HERE))
 
 from oracle import bv_oracle as O  # noqa: E402
-from big_vision_b200.models.proj.image_text import two_towers  # noqa: E402
 import common  # noqa: E402
 
 
 def main():
-  model = two_towers.Model(**common.TINY)
-  P = model.init(0, common.TINY_IMAGE_SHAPE, common.TINY_TEXT_SHAPE, device="cpu")
-  tree = P.numpy_tree("f")
-  image, text = common.synthetic_batch(common.TINY_IMAGE_SHAPE, common.TINY_TEXT_SHAPE,
-                                       common.TINY["text"]["vocab_size"])
-  out = {"image": image, "text": text}
-  for k, v in tree.items():
-    out["param:" + k] = v.astype(np.float32)
+  tree, image, text = common.tiny_inputs()
+  out = {"text": text, "params_sha256": np.array(common.sha256_of(tree)),
+         "image_sha256": np.array(common.sha256_of({"image": image}))}
   cfg = common.oracle_cfg(common.TINY)
   for mm in ("float32", "bfloat16"):
     loss, grads, zimg, ztxt = O.siglip_value_and_grad(tree, image, text, cfg, mm)

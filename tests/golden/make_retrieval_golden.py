@@ -1,16 +1,21 @@
 """Generates tests/golden/retrieval.npz by RUNNING THE REFERENCE's own (numpy-only) retrieval metric
-code (big_vision/evaluators/proj/image_text/image_text_retrieval.py) in this container on seeded
-random distance matrices without ties.  /root/reference is not available on the GPU box, so the
-outputs are committed.
+code (big_vision/evaluators/proj/image_text/image_text_retrieval.py) on seeded random distance
+matrices without ties.  The tests do not need the reference: its outputs are committed.
 
-  python tests/golden/make_retrieval_golden.py
+  python tests/golden/make_retrieval_golden.py <directory holding the big_vision package>
+
+Each matrix is stored as the rank of every distance among all distances of that matrix (uint32, which
+compresses to well under 1 MB); the matrix the reference ran on is
+(rank * (2 / rank.size)).astype(float32), as tests/test_eval_paths.py rebuilds it.
 """
 import os
 import sys
 
 import numpy as np
 
-sys.path.insert(0, "/root/reference")
+if len(sys.argv) != 2:
+  sys.exit(__doc__)
+sys.path.insert(0, sys.argv[1])
 from big_vision.evaluators.proj.image_text import image_text_retrieval as ref  # noqa: E402
 
 out = {}
@@ -25,16 +30,16 @@ for name, (ni, per) in {"a": (50, 5), "b": (333, 1), "c": (200, 5)}.items():
   zi_n = zi / np.linalg.norm(zi, axis=1, keepdims=True)
   zt_n = zt / np.linalg.norm(zt, axis=1, keepdims=True)
   d64 = 1.0 - zi_n.astype(np.float64) @ zt_n.astype(np.float64).T
-  # replace every distance by its global rank scaled into (0, 2): same order, and all values are
+  # replace every distance by its global rank scaled into [0, 2): same order, and all values are
   # distinct float32 numbers, so the reference's (unstable) argsort has a unique answer
-  order = np.argsort(d64, axis=None, kind="stable")
-  d = np.empty(d64.size, np.float32)
-  d[order] = (np.arange(d64.size, dtype=np.float64) * (2.0 / d64.size)).astype(np.float32)
-  d = d.reshape(d64.shape)
+  rank = np.empty(d64.size, np.uint32)
+  rank[np.argsort(d64, axis=None, kind="stable")] = np.arange(d64.size, dtype=np.uint32)
+  rank = rank.reshape(d64.shape)
+  d = (rank.astype(np.float64) * (2.0 / rank.size)).astype(np.float32)
   assert len(np.unique(d)) == d.size, "ties would make the reference's argsort order ambiguous"
   t2i = ref.text_to_image_retrieval_eval(d, list(corr))
   i2t = ref.image_to_text_retrieval_eval(d, list(corr))
-  out[f"{name}_dist"] = d
+  out[f"{name}_rank"] = rank
   out[f"{name}_corr"] = corr.astype(np.int32)
   out[f"{name}_t2i"] = np.array([t2i[f"Recall@{k}"] for k in ref.RECALL_THRESHOLDS], np.float64)
   out[f"{name}_i2t"] = np.array([i2t[f"Recall@{k}"] for k in ref.RECALL_THRESHOLDS], np.float64)

@@ -116,6 +116,30 @@ def test_bench_refuses_to_run_the_product_arm_without_a_gpu():
   assert r.returncode != 0 and r.stdout.strip() == "" and "needs a GPU" in r.stderr
 
 
+@pytest.mark.gpu
+def test_bench_dumps_what_the_last_timed_step_returned(tmp_path):
+  """`bench.py --dump-outputs DIR`: the last timed step's measurements, the optimizer's step count (warm-up +
+  --steps updates, so --steps sets the timed steps) and a fixed sample of the train state, as float32 /
+  float64 .npy files of at most 64 MB in all."""
+  import json
+  import subprocess
+  import sys
+  import numpy as np
+  r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "2", "--warmup", "3",
+                      "--per-gpu-batch", "64", "--no-cpu-baseline", "--no-gpu-baseline",
+                      "--dump-outputs", str(tmp_path)], capture_output=True, text=True, timeout=900)
+  assert r.returncode == 0, r.stderr[-2000:]
+  line = json.loads(r.stdout.strip().splitlines()[-1])
+  out = {p.stem: np.load(p) for p in tmp_path.iterdir()}
+  assert set(out) == {"training_loss", "l2_grads", "l2_params", "l2_updates", "opt_count",
+                      "params", "grads", "adam_mu", "adam_nu"}
+  assert sum(p.stat().st_size for p in tmp_path.iterdir()) <= 64 << 20
+  assert all(a.dtype in (np.float32, np.float64) and np.isfinite(a).all() for a in out.values())
+  assert float(out["opt_count"]) == line["warmup"] + line["steps"] == 5
+  assert out["params"].shape == out["grads"].shape == out["adam_mu"].shape == out["adam_nu"].shape == (1 << 21,)
+  assert float(out["training_loss"]) > 0 and float(out["l2_params"]) > 0 and np.any(out["grads"] != 0)
+
+
 def test_reference_arm_prints_the_contract_line():
   """`bench.py --impl reference`: the oracle port on the host cores, one JSON line with the same metric /
   unit / config keys as the product arm plus impl, cpu_baseline and an e2e block with zero copies."""

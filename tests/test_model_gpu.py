@@ -1,7 +1,6 @@
 """GPU parity of the whole SigLIP step (two towers + pairwise sigmoid loss + backward + Adam)
 through the product's public API against the oracle and the committed golden vectors."""
 import math
-import os
 
 import numpy as np
 import pytest
@@ -11,7 +10,6 @@ import common
 from oracle import bv_oracle as O
 
 pytestmark = pytest.mark.gpu
-GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "siglip_tiny.npz")
 
 
 def _relerr(a, b):
@@ -22,13 +20,12 @@ def _relerr(a, b):
 @pytest.fixture(scope="module")
 def tiny():
   from big_vision_b200.models.proj.image_text import two_towers
-  z = np.load(GOLD)
+  z, tree, image, text = common.load_golden_tiny()
   model = two_towers.Model(**common.TINY)
   P = model.init(0, common.TINY_IMAGE_SHAPE, common.TINY_TEXT_SHAPE, device="cuda")
-  tree = {k[len("param:"):]: z[k] for k in z.files if k.startswith("param:")}
   P.load_tree(tree)
-  image = torch.from_numpy(z["image"]).cuda()
-  text = torch.from_numpy(z["text"]).cuda()
+  image = torch.from_numpy(image).cuda()
+  text = torch.from_numpy(text).cuda()
   return model, P, image, text, z, tree
 
 

@@ -12,7 +12,6 @@ import common
 from oracle import bv_oracle as O
 
 F64 = torch.float64
-GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "siglip_tiny.npz")
 
 
 def test_layer_norm_matches_torch():
@@ -91,10 +90,9 @@ def test_adam_reference_first_step_is_sign_update():
 
 
 def test_golden_vectors_reproduce():
-  z = np.load(GOLD)
-  tree = {k[len("param:"):]: z[k] for k in z.files if k.startswith("param:")}
+  z, tree, image, text = common.load_golden_tiny()
   cfg = common.oracle_cfg(common.TINY)
-  loss, grads, zimg, ztxt = O.siglip_value_and_grad(tree, z["image"], z["text"], cfg, "float32")
+  loss, grads, zimg, ztxt = O.siglip_value_and_grad(tree, image, text, cfg, "float32")
   assert loss == pytest.approx(float(z["float32:loss"]), rel=1e-9)
   assert np.allclose(zimg, z["float32:zimg"], atol=1e-9)
   for k in ("t", "b", "img/MAPHead_0/probe", "txt/Embed_0/embedding",
@@ -103,10 +101,10 @@ def test_golden_vectors_reproduce():
 
 
 def test_golden_inputs_follow_the_synthetic_recipe():
-  z = np.load(GOLD)
+  z = np.load(common.GOLDEN_TINY)
   image, text = common.synthetic_batch(common.TINY_IMAGE_SHAPE, common.TINY_TEXT_SHAPE,
                                        common.TINY["text"]["vocab_size"])
-  assert np.array_equal(image, z["image"]) and np.array_equal(text, z["text"])
+  assert common.sha256_of({"image": image}) == str(z["image_sha256"]) and np.array_equal(text, z["text"])
   assert (text[:, -1] == 1).all() and image.min() >= -1 and image.max() <= 1
 
 

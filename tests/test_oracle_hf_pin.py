@@ -167,19 +167,17 @@ def test_oracle_gradients_match_transformers_siglip(pair):
 
 def test_committed_golden_vectors_equal_transformers_outputs():
   """tests/golden/siglip_tiny.npz is what the GPU parity tests (tests/test_model_gpu.py) compare the CUDA path
-  with.  It was written by the oracle (tests/golden/make_golden.py); here its parameters and inputs go
-  through transformers' SiglipModel and must reproduce the file's float32-mode embeddings, loss and every
+  with.  It was written by the oracle (tests/golden/make_golden.py); here the parameters and inputs it was
+  computed from go through transformers' SiglipModel and must reproduce the file's float32-mode embeddings, loss and every
   stored gradient -- which ties the GPU tests' reference values to an implementation other than the oracle."""
-  import os
   import common
-  z = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "siglip_tiny.npz"))
-  tree = {k[len("param:"):]: z[k] for k in z.files if k.startswith("param:")}
+  z, tree, image, text = common.load_golden_tiny()
   kw = common.TINY
   hf = _hf_model(tree, kw["image"]["width"], kw["image"]["depth"], kw["image"]["mlp_dim"], kw["image"]["num_heads"],
                  common.TINY_IMAGE_SHAPE[1], kw["image"]["patch_size"][0], kw["text"]["vocab_size"],
                  common.TINY_TEXT_SHAPE[1], kw["out_dim"][1])
-  image = torch.from_numpy(z["image"]).double().permute(0, 3, 1, 2)
-  out = hf(input_ids=torch.from_numpy(z["text"]).long(), pixel_values=image, return_loss=True)
+  image = torch.from_numpy(image).double().permute(0, 3, 1, 2)
+  out = hf(input_ids=torch.from_numpy(text).long(), pixel_values=image, return_loss=True)
   assert float((out.image_embeds.detach() - torch.from_numpy(z["float32:zimg"])).abs().max()) < 1e-7
   assert float((out.text_embeds.detach() - torch.from_numpy(z["float32:ztxt"])).abs().max()) < 1e-7
   assert float(out.loss) == pytest.approx(float(z["float32:loss"]), rel=1e-7)
